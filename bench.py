@@ -6,7 +6,10 @@ hypotheses, fold, delay-spread, argmax, signal power) over one batch of syntheti
 buffers.  Workload = BASELINE.json configs[1]: 153600-sample capture buffers, +-100 ppm grid at
 739 MHz (n_f = 31), ds_comb_arm 2, synthetic rtl-sdr-like 8-bit IQ (SURVEY.md 8d).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl b200|reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned, for a fixed sample of its buffers, as DIR/<name>.npy, so
+that two builds run with the same arguments (hence the same seeded inputs) can be compared output for output.
 
 Launch for N>1:  python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N
 Capture buffers shard across ranks with no data-path collective (weak scaling: B buffers per
@@ -39,6 +42,8 @@ PPM = 100.0
 ARM = 2
 FS = 1.92e6
 SEED0 = 0xC0FFEE
+DUMP_SEED = 0xD0
+DUMP_BYTES = 32e6                  # room for 8 whole buffers of the n_f = 31 workload, half the 64 MB a dump may take
 
 
 def synth_cu8(seed, n_cap=N_CAP, sigma=20.0):
@@ -321,6 +326,22 @@ def all_max(torch, dist, world, dev, v):
     return float(t.item())
 
 
+def dump_outputs(out_dir, torch, single, pw, frq, spi):
+    """Write the outputs lcs_xcorr_pss_device returned for a seeded sample of the batch's buffers, in the layout it writes:
+    single [b][3][n_f][9600] float32, pow and frq [b][3][9600] (frq as float32, exact for frequency indices),
+    sp_incoherent [b][9600] float64.  Returns the sampled buffer indices."""
+    B, _, n_f, _ = single.shape
+    per_buf = 9600 * (3 * n_f * 4 + 3 * 8 + 3 * 4 + 8)
+    n = max(1, min(B, int(DUMP_BYTES // per_buf)))
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(B, n, replace=False))
+    sel = torch.from_numpy(idx).to(single.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t, dt in (("single", single, np.float32), ("pow", pw, np.float64), ("frq", frq, np.float32),
+                        ("sp_incoherent", spi, np.float64)):
+        np.save(os.path.join(out_dir, name + ".npy"), t.index_select(0, sel).cpu().numpy().astype(dt))
+    return idx
+
+
 def sweep_leg(L, torch, dist, ctx, rank, world, dev, barrier, reps=3):
     """BASELINE config 4: 512-channel frequency sweep (715.0 MHz + k*100 kHz, CellSearch.cpp:465), one capture buffer per
     channel (synthetic 8-bit IQ; channel 240 = 739.0 MHz carries the reference's real capture), channels round-robin over
@@ -420,7 +441,14 @@ def main():
     ap.add_argument("--no-extra-legs", action="store_true", help="skip the sweep / tracker / search legs (ncu captures)")
     ap.add_argument("--workload", default="search", choices=["search", "tracker"],
                     help="search: BASELINE configs[1] (n_f=31); tracker: SURVEY 8d config 5 shape (n_f=1 at the tracked offset)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write single / pow / frq / sp_incoherent of the last timed step (rank 0, a seeded sample of its "
+                         "buffers) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -513,6 +541,12 @@ def main():
     ms_max = all_max(torch, dist, world, dev, ms)
     capbufs_per_s = world * B * args.steps / (ms_max / 1e3)
     value = capbufs_per_s * N_CAP / 1e6
+    r_last = (args.warmup + args.steps - 1) % ring      # ring slot the last timed step wrote
+
+    dump = None
+    if rank == 0 and args.dump_outputs:
+        idx = dump_outputs(args.dump_outputs, torch, d_single[r_last], d_pow[r_last], d_frq[r_last], d_spi[r_last])
+        dump = {"dir": os.path.abspath(args.dump_outputs), "ring_slot": r_last, "buffers": idx.tolist()}
 
     # ---- parity spot check: one buffer of the LAST timed step against the oracle (test infrastructure, after the timing) ----
     parity = None
@@ -521,7 +555,6 @@ def main():
         import lcs_oracle as O
         os.sched_setaffinity(0, orig_affinity)          # the CPU oracle may use every host core
         O.set_threads(host_threads())
-        r_last = (args.warmup + args.steps - 1) % ring
         b_chk = B // 2
         cu8 = d_iq[r_last][b_chk].cpu().numpy()
         ref = O.xcorr_pss(((cu8.astype(np.float64) - 127) / 128).view(np.complex128).reshape(-1), f, ARM, FC, FC, FS, want_sp=False)
@@ -658,6 +691,8 @@ def main():
             line["e2e_search"] = search
         if parity is not None:
             line["parity_spot"] = parity
+        if dump is not None:
+            line["dump_outputs"] = dump
         if sweep_res is not None:
             line["sweep"] = sweep_res
         if tracker_res is not None:
